@@ -5,11 +5,11 @@
     python bench.py --impl reference --gpus N --steps K ...  # the reference algorithm on host cores (oracle port)
 
 A step is one pass of the hot path over one batch: 1 000 000 synthetic XYZRGBA points (16 B each) inserted into the
-growing octree by kernel_construct. The workload does NOT depend on --steps: at N = 1 it is BASELINE.json configs[2],
-the 350 M-point stream (Morro-Bay stand-in terrain, no dataset on the box), inserted from a freshly reset octree in
-350 spatially coherent 1 M-point batches; a timed PASS is the whole stream, the reported time is the median of
->= 5 passes from reset (SURVEY.md §8d), and ms_per_step is that time per 1 M-point batch. --steps only echoes into the
-line (and bounds the reference arm's CPU sample), --warmup batches are inserted untimed first.
+growing octree by kernel_construct. The stream is BASELINE.json configs[2], the 350 M-point scan (Morro-Bay stand-in
+terrain, generated), inserted from a freshly reset octree in spatially coherent 1 M-point batches. A timed PASS inserts
+the first K = --steps batches of that stream (all 350 with --steps 350), the reported time is the median of >= 5 passes
+from reset (SURVEY.md §8d), and ms_per_step is that time per 1 M-point batch; --warmup batches are inserted untimed
+first. --dump-outputs DIR writes the octree the last timed pass built (canonical form, DESIGN.md §3) as .npy files.
 
 With N > 1 every rank owns a complete builder and inserts its own 350 M-point scan tile of the same extent and density
 (tile g of a survey of N tiles): per-GPU work is identical to N = 1, scaling is weak, and there is no data-path
@@ -68,6 +68,7 @@ def parse():
     ap.add_argument("--no-render", action="store_true")
     ap.add_argument("--no-reference-gpu", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the LAS / file-streamer / config-4 legs")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the octree of the last timed pass to DIR/*.npy")
     return ap.parse_args()
 
 
@@ -402,6 +403,21 @@ def bench_stream_file(sim_device, host_batches, mn, mx):
     return out
 
 
+def dump_outputs(sim, out_dir):
+    """What a caller of the timed path receives, reduced to what is the same from run to run (DESIGN.md §3): the
+    deterministic Stats fields and the octree's canonical form (per node, in (level, X, Y, Z) order: counters, chunk
+    counts, and the hashes of its sorted points and voxel positions as 32-bit halves), all exact in float64."""
+    import oracle
+    os.makedirs(out_dir, exist_ok=True)
+    st = sim.stats()
+    rec = oracle.canon_from_image(*sim.download_octree()).records
+    cols = ("level", "X", "Y", "Z", "counter", "numPoints", "numVoxels", "numVoxelsStored", "isLeaf", "chunksPoints", "chunksVoxels")
+    halves = [(rec[f] >> np.uint64(s)) & np.uint64(0xFFFFFFFF) for f in ("hashPoints", "hashVoxelPos") for s in (32, 0)]
+    np.save(os.path.join(out_dir, "stats.npy"), np.array([int(getattr(st, f)) for f in oracle.STATS_FIELDS], dtype=np.float64))
+    np.save(os.path.join(out_dir, "octree_nodes.npy"), np.stack([rec[c].astype(np.float64) for c in cols], axis=1))
+    np.save(os.path.join(out_dir, "octree_hashes.npy"), np.stack([h.astype(np.float64) for h in halves], axis=1))
+
+
 def run_reference(args, rank, world):
     """The reference's algorithm on the host cores: oracle port (the reference has no CPU octree builder to compile; its
     kernels need a GPU). Same workload (the 350 M-point stream of the numpy generator the device generator restates
@@ -555,15 +571,16 @@ def main():
             dist.barrier()
         torch.cuda.synchronize()
 
-    W, K = max(args.warmup, 0), args.steps
     NB = args.batches
+    W, K = max(args.warmup, 0), min(max(args.steps, 1), NB)
     passes = max(args.passes, 1)
-    npts = NB * BATCH
+    npts = K * BATCH                                         # timed points per pass: the first K batches of the stream
+    nb_gen = max(K, min(W, NB), min(16, NB))                 # batches generated: timed, warm-up and the CPU legs' sample
     mn, mx = (0.0, 0.0, 0.0), data.TERRAIN_EXTENT
     peak, peak_src = peaks()
 
     import oracle          # the reference kernels' scratch needs 408.8 MB of momentary buffer; ours fits 300 MB either way
-    sim = SimLOD(W_PX, H_PX, device=local_rank, persistent_bytes=max(8 << 30, NB * (72 << 20)))
+    sim = SimLOD(W_PX, H_PX, device=local_rank, persistent_bytes=max(8 << 30, K * (72 << 20)))
     sampler = ClockSampler(local_rank)
     sampler.start()
     windows = []
@@ -571,8 +588,8 @@ def main():
         sim.set_box(mn, mx)
         # this rank's stream (tile `rank` of the survey), generated on the device; a pinned host copy for the e2e leg
         t_gen = time.time()
-        dptr = sim.device_alloc(npts * 16)
-        sim.generate(sim.GEN_TERRAIN, dptr, npts, 0, npts, TERRAIN_SEED + rank)
+        dptr = sim.device_alloc(nb_gen * BATCH * 16)
+        sim.generate(sim.GEN_TERRAIN, dptr, NB * BATCH, 0, nb_gen * BATCH, TERRAIN_SEED + rank)
         host_ptr = sim.host_alloc(npts * 16)
         numa_node = sim.numa_node()
         sim._check(sim._lib.simlod_memcpy_dtoh(sim._ctx, host_ptr, dptr, npts * 16))
@@ -596,13 +613,15 @@ def main():
         t_value = sdist.max_over_ranks(float(np.median(ts)), dev)
         t_kernel = sdist.max_over_ranks(kernel_ms, dev)
         totals = sdist.reduce_stats(st, dev)
+        if args.dump_outputs and rank == 0:
+            dump_outputs(sim, args.dump_outputs)
 
         # ---- render on the built octree (rank-local; reported at rank 0) --------------------------
         render = None
         if not args.no_render and rank == 0:
             t0 = time.time()
             render = render_sweep(sim, mx, peak)
-            render["metric"] = "render Msamples/s @1GPU (1920x1080), 6 cameras on the %d M-point octree" % NB
+            render["metric"] = "render Msamples/s @1GPU (1920x1080), 6 cameras on the %d M-point octree" % K
             render["render_blocks"] = sim.launch_info()["render_blocks"]
             windows.append((t0, time.time()))
 
@@ -610,7 +629,7 @@ def main():
         reference_gpu = None
         if rank == 0 and world == 1 and not args.no_reference_gpu:
             t0 = time.time()
-            reference_gpu = bench_reference_gpu(local_rank, dptr, NB, (mn, mx), peak, sim)
+            reference_gpu = bench_reference_gpu(local_rank, dptr, K, (mn, mx), peak, sim)
             windows.append((t0, time.time()))
             reference_gpu["clocks"] = sampler.summary([windows[-1]])
 
@@ -639,7 +658,7 @@ def main():
         # a bounded host sample of the same stream for the CPU legs (rank 0, N = 1)
         sample_batches = []
         if rank == 0 and world == 1:
-            nb_s = min(16, NB)
+            nb_s = min(16, nb_gen)
             raw = sim.memcpy_dtoh(dptr, nb_s * BATCH * 16).view(data.POINT_DTYPE)
             sample_batches = [raw[i * BATCH:(i + 1) * BATCH] for i in range(nb_s)]
         # ---- one octree over the N GPUs (SURVEY.md §8f-3), N > 1 only ----------------------------------------
@@ -648,7 +667,7 @@ def main():
             t0 = time.time()
             try:
                 sim.set_box(mn, mx)
-                merged = bench_merged_octree(sim, dptr, NB, rank, world, dev, barrier)
+                merged = bench_merged_octree(sim, dptr, nb_gen, rank, world, dev, barrier)
             except Exception as e:
                 merged = {"error": repr(e)}
             windows.append((t0, time.time()))
@@ -713,15 +732,15 @@ def main():
         v_frac = voxels_total / npts
         alg_bytes = (32.0 + 32.0 * s_frac + 16.0 * v_frac) * npts          # this rank, one pass
         achieved = alg_bytes / (kernel_ms * 1e-3) / 1e9
-        traffic = recorded_traffic(NB)
+        traffic = recorded_traffic(K)
         n_launch = max(launches_per_pass, 1)
         line = {
             "metric": METRIC, "value": round(value, 2), "unit": "Mpoints/s", "n_gpus": world, "steps": K, "warmup": W,
-            "ms_per_step": round(t_value / NB, 5), "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
+            "ms_per_step": round(t_value / K, 5), "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
             "dtype": "u32+f32", "data": "synthetic",
             "config": {"workload": workload_name(NB),
-                       "batch_points": BATCH, "points_per_gpu": npts, "steps_per_pass": NB, "timed_passes": passes,
-                       "timing": "median of %d passes, each the whole stream from reset (a step = one 1M-point batch; --steps does not size the workload); max over ranks of the per-rank median" % passes,
+                       "batch_points": BATCH, "points_per_gpu": npts, "steps_per_pass": K, "timed_passes": passes,
+                       "timing": "median of %d passes, each the first %d batches of the %d-batch stream from reset (a step = one 1M-point batch); max over ranks of the per-rank median" % (passes, K, NB),
                        "parallelism": "batch-sharded x%d (one %d-batch scan tile per GPU, no data-path collective)" % (world, NB),
                        "l2": "inputs %d MB > L2 (126 MB); L2 flushed before each timed pass" % (npts * 16 // 1000000),
                        "kernel_only_mpoints_per_s": round(all_pts / t_kernel / 1e3, 2),
@@ -739,7 +758,7 @@ def main():
                          "avg_launch_ms": round(kernel_ms / n_launch, 4), "algorithmic_bytes_per_launch": round(alg_bytes / n_launch),
                          "note": "latency/atomic bound, not bandwidth bound: see DESIGN.md §7"},
             "e2e": {"value": round(all_pts / t_e2e / 1e3, 2), "unit": "Mpoints/s", "h2d_bytes_per_step": BATCH * 16,
-                    "d2h_bytes_per_step": round(112.0 * (e_launches + 1) / NB, 1), "wall_clock_value": round(all_pts / t_e2e_wall / 1e3, 2),
+                    "d2h_bytes_per_step": round(112.0 * (e_launches + 1) / K, 1), "wall_clock_value": round(all_pts / t_e2e_wall / 1e3, 2),
                     "launches": e_launches, "passes": e_passes, "pinned_on_numa_node": numa_node},
             "gpu_launches": launches_per_pass * passes,
             "clocks": sampler.summary(windows),
